@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- queries/sec of predict() on the BASELINE.json workload (see DESIGN.md "Measurement").
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 ... bench.py --gpus N ...
 
 A step = one predict pass (E encoder -> K prototype kNN -> H head -> blend, top-5 labels) over one batch of
@@ -13,6 +13,9 @@ One JSON line on rank 0.  Before the timed region the step's kNN result of 16 qu
 At N = 1 the line also carries sub-results measured after the headline (never inside its timed region): `k_equals_C`
 (predict() semantics, k = 1000), `cfg4` (BASELINE configs[3], the add_examples loop), `gpu_library_baseline` (HF BertModel in
 torch eager on the same GPU) and `cpu_baseline` (the oracle port on the host cores).
+--dump-outputs DIR writes what the last timed step returned (top-5 class ids and scores of every query of this rank) as
+DIR/top5_classes.npy (float64) and DIR/top5_scores.npy (float32); at N > 1 each rank writes its own, suffixed _rank<r>.  Every
+input is seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -305,7 +308,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true", help=argparse.SUPPRESS)
     ap.add_argument("--no-extras", action="store_true", help="skip the sub-results (k = C, cfg4, HF-eager comparator)")
     ap.add_argument("--cfg4-examples", type=int, default=50_000, help=argparse.SUPPRESS)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's top-5 class ids and scores as DIR/<name>.npy (B200 path only)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs records the B200 path's outputs; it does not apply to --impl reference")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -412,14 +421,14 @@ def main():
         t0 = time.time()
         e0.record()
         for _ in range(steps):
-            fn()
+            out = fn()
         e1.record()
         torch.cuda.synchronize(); barrier()
         t1 = time.time()
         ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
         if G > 1:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
-        return float(ms.item()), t0, t1
+        return float(ms.item()), t0, t1, out
 
     # ---- warm-up, shape sanity and the parity check of this very step (outside the timed region)
     for _ in range(args.warmup):
@@ -459,15 +468,22 @@ def main():
         time.sleep(0.3)
     _cabi.profile_enable(True)
     l0 = _cabi.launch_count()
-    ms, t0, t1 = timed(step_device, args.steps)
+    ms, t0, t1, last = timed(step_device, args.steps)
     launches = _cabi.launch_count() - l0
     _cabi.profile_enable(False)
     prof = {c: _cabi.profile_read(c) for c in range(5)}
     clocks = sampler.stop(t0, t1) if rank == 0 else None
     kstats = pipe.knn_stats(reset=True)
+    if args.dump_outputs:
+        # copied before anything else runs: the step returns views of the pipeline's output buffers
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        sfx = f"_rank{rank}" if G > 1 else ""
+        np.save(os.path.join(args.dump_outputs, f"top5_classes{sfx}.npy"), last[0].cpu().numpy().astype(np.float64))
+        np.save(os.path.join(args.dump_outputs, f"top5_scores{sfx}.npy"), last[1].cpu().numpy().astype(np.float32))
     for _ in range(2):
         step_host()
-    ms_e2e, _, _ = timed(step_host, args.steps)
+    ms_e2e, _, _, _ = timed(step_host, args.steps)
     # the scan kernel by itself (same queries, same shard, nothing else on the GPU): inside the step it shares the SMs with the head
     # forward on the side stream, which is what `ms_per_launch` above includes
     knn_alone_ms = None

@@ -11,8 +11,8 @@ Fixtures
   golden_router.npz      the two real prototypes of scripts/adaptive_router/tensors.safetensors (6 KB,
                          inter-prototype d = 0.001965: near-tie stress) + reference search results
   golden_head.npz        AdaptiveHead forward / EWC loss values of the reference on seeded inputs
-  golden_classifier.npz  tiny seeded BERT checkpoint + vocab, reference _get_embeddings / add_examples /
-                         predict / predict_batch outputs and the reference-trained head
+  golden_classifier.npz  digest + vocab of the tiny seeded BERT checkpoint (oracle/tiny_bert.py rebuilds it), reference
+                         _get_embeddings / add_examples / predict / predict_batch outputs and the reference-trained head
   golden_training.npz    the reference's two training loops (_train_adaptive_head, _train_new_classes + EWC/Fisher)
                          run UNMODIFIED with recorders hooked onto torch/numpy entry points: the dataset of every
                          training call, every batch index list the DataLoader yielded, np.random.choice draws,
@@ -33,6 +33,8 @@ ROOT = os.path.dirname(HERE)
 sys.path.insert(0, os.path.join(HERE, "shim"))
 sys.path.insert(0, "/root/reference/src")
 sys.path.insert(0, ROOT)
+from oracle import tiny_bert  # noqa: E402
+
 OUT = os.path.join(ROOT, "tests", "golden")
 
 
@@ -164,7 +166,6 @@ def gen_classifier():
     p1l, p1s = pack(pred_k1, 1)
     pbl, pbs = pack(pred_b, 2)
     head_sd = {("head_" + k): v.detach().numpy() for k, v in clf.adaptive_head.state_dict().items()}
-    model_sd = {("bert_" + k): v.detach().numpy() for k, v in model.state_dict().items()}
     protos = np.stack([clf.memory.prototypes[l].numpy() for l in sorted(clf.memory.prototypes)])
     np.savez_compressed(
         os.path.join(OUT, "golden_classifier.npz"),
@@ -174,39 +175,15 @@ def gen_classifier():
         training_history=json.dumps(clf.training_history), train_steps=clf.train_steps,
         pred_labels=pl, pred_scores=ps, pred_k1_labels=p1l, pred_k1_scores=p1s, predb_labels=pbl, predb_scores=pbs,
         train_top1=np.array([label_names.index(l) for l in train_top1]),
-        bert_config=json.dumps(cfg.to_dict()), **head_sd, **model_sd)
+        bert_config=json.dumps(cfg.to_dict()), bert_sha256=tiny_bert.digest(model.state_dict()), **head_sd)
     print("golden_classifier ok; labels", label_names, "pred[0]", pred[0])
 
 
-def _tiny_checkpoint(hidden=128):
-    """seeded 2-layer BERT + synthetic vocab on disk (same recipe as gen_classifier)"""
-    from transformers import BertConfig, BertModel, BertTokenizerFast
-    words = [f"w{i}" for i in range(195)]
-    vocab = ["[PAD]", "[UNK]", "[CLS]", "[SEP]", "[MASK]"] + words
-    cfg = BertConfig(vocab_size=len(vocab), hidden_size=hidden, num_hidden_layers=2, num_attention_heads=2,
-                     intermediate_size=2 * hidden, max_position_embeddings=64, type_vocab_size=2, pad_token_id=0)
-    torch.manual_seed(1234)
-    model = BertModel(cfg)
-    g = torch.Generator().manual_seed(99)
-    with torch.no_grad():
-        for n, p in model.named_parameters():
-            if "LayerNorm" in n or n.endswith(".bias"):
-                p.add_(0.1 * torch.randn(p.shape, generator=g))
-            elif "weight" in n and p.dim() == 2:
-                # word embeddings x4: token identity survives to the CLS row, so the classes are learnable (nearest-centroid
-                # accuracy 0.93 on the sentences below) and the loops do not early-stop at once
-                p.mul_(4.0 if "word_embeddings" in n else 3.0)
-        # ... and the constant part of the CLS row's input ([CLS] word row, position 0, token types) is zeroed, otherwise every
-        # sentence embeds within 0.2 of every other one and 10 epochs of lr 1e-3 learn nothing (mean pair distance 1.14 now)
-        model.embeddings.word_embeddings.weight[2].zero_()
-        model.embeddings.position_embeddings.weight[0].zero_()
-        model.embeddings.token_type_embeddings.weight.zero_()
-    tmp = tempfile.mkdtemp(prefix="golden_ckpt_")
-    model.save_pretrained(tmp)
-    # transformers 5.x: BertTokenizerFast(vocab_file=...) silently keeps only the special tokens (every word -> [UNK]);
-    # the vocabulary has to be passed as a dict
-    BertTokenizerFast(vocab={w: i for i, w in enumerate(vocab)}, do_lower_case=True).save_pretrained(tmp)
-    return tmp, words, vocab, model, cfg
+def _tiny_checkpoint():
+    """the seeded tiny BERT of oracle/tiny_bert.py + its vocab on disk"""
+    model, cfg = tiny_bert.build()
+    tmp = tiny_bert.save_checkpoint(model, tempfile.mkdtemp(prefix="golden_ckpt_"))
+    return tmp, tiny_bert.WORDS, tiny_bert.VOCAB, model, cfg
 
 
 class _Recorder:
@@ -458,8 +435,7 @@ def gen_training():
     out["ml_thresholds"] = np.array(json.dumps(ml.label_thresholds))
     out["bert_config"] = np.array(json.dumps(clf.model.config.to_dict()))
     out["vocab"] = np.array(vocab)
-    for k, v in clf.model.state_dict().items():
-        out["bert_" + k] = v.detach().numpy()
+    out["bert_sha256"] = np.array(tiny_bert.digest(clf.model.state_dict()))
     np.savez_compressed(os.path.join(OUT, "golden_training.npz"), **out)
     print("golden_training ok: h3 steps", len(out["h3_loss"]), "epochs", len(out["h3_steps_per_epoch"]),
           "| h4 steps", len(out["h4_loss"]), "epochs", len(out["h4_steps_per_epoch"]), "rows", out["h4_X"].shape,

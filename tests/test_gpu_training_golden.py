@@ -87,16 +87,10 @@ def test_product_batch_order_is_the_dataloaders(g):
 
 @pytest.fixture(scope="module")
 def ckpt_dir(g):
-    from transformers import BertConfig, BertModel, BertTokenizerFast
-    d = tempfile.mkdtemp(prefix="golden_train_ckpt_")
-    cfg = BertConfig(**{k: v for k, v in json.loads(str(g["bert_config"])).items()
-                        if k in ("vocab_size", "hidden_size", "num_hidden_layers", "num_attention_heads",
-                                 "intermediate_size", "max_position_embeddings", "type_vocab_size", "pad_token_id")})
-    m = BertModel(cfg)
-    m.load_state_dict({k[5:]: torch.from_numpy(g[k]) for k in g.files if k.startswith("bert_") and k != "bert_config"})
-    m.save_pretrained(d)
-    BertTokenizerFast(vocab={w: i for i, w in enumerate(g["vocab"].tolist())}, do_lower_case=True).save_pretrained(d)
-    return d
+    from oracle import tiny_bert
+    assert g["vocab"].tolist() == tiny_bert.VOCAB
+    m, _ = tiny_bert.model(g["bert_sha256"])
+    return tiny_bert.save_checkpoint(m, tempfile.mkdtemp(prefix="golden_train_ckpt_"))
 
 
 def test_add_examples_end_to_end_follows_the_reference_run(acb, g, ckpt_dir, monkeypatch):
