@@ -23,7 +23,7 @@ AC_KNN_MAX_K = 2048
 AC_KNN_TENSOR_MAX_K = 1024
 AC_ACT_LOGITS, AC_ACT_SOFTMAX, AC_ACT_SIGMOID = 0, 1, 2
 AC_LOSS_CE, AC_LOSS_BCE = 0, 1
-AC_ARCH_BERT, AC_ARCH_ROBERTA = 0, 1
+AC_ARCH_BERT, AC_ARCH_ROBERTA, AC_ARCH_MODERNBERT = 0, 1, 2
 AC_PREC_TF32, AC_PREC_F16 = 0, 1
 
 EXPORTS = [
@@ -31,7 +31,7 @@ EXPORTS = [
     "ac_knn_workspace_bytes", "ac_knn_l2_topk", "ac_knn_make_shadow", "ac_row_sqnorm", "ac_topk_merge", "ac_proto_scores",
     "ac_segment_mean", "ac_memory_append_prune",
     "ac_head_forward", "ac_head_train_workspace_bytes", "ac_head_train_step", "ac_head_train_epoch", "ac_head_phase_timing", "ac_head_train_plan", "ac_head_grad", "ac_ewc_penalty",
-    "ac_encoder_create", "ac_encoder_destroy", "ac_encoder_forward_cls", "ac_encoder_last_hidden", "ac_linear_tc",
+    "ac_encoder_create", "ac_encoder_create_modernbert", "ac_encoder_destroy", "ac_encoder_forward_cls", "ac_encoder_last_hidden", "ac_linear_tc",
     "ac_proto_class_scores", "ac_proto_class_scores_n", "ac_blend_dense", "ac_topk_desc_workspace_bytes", "ac_topk_desc", "ac_blend_topk",
     "ac_pipeline_create", "ac_pipeline_destroy", "ac_pipeline_predict_device", "ac_pipeline_predict_host",
     "ac_pipeline_encode", "ac_pipeline_embeddings", "ac_pipeline_search_shard", "ac_pipeline_finish_sharded",
@@ -76,6 +76,21 @@ class EncoderWeights(Structure):
                 ("out_ln_w", _PP), ("out_ln_b", _PP)]
 
 
+class ModernBertEncoderConfig(Structure):
+    _fields_ = [("layers", c_int), ("hidden", c_int), ("heads", c_int), ("intermediate", c_int), ("vocab", c_int),
+                ("norm_eps", c_float), ("precision", c_int), ("max_tokens", c_int), ("cls_only", c_int),
+                ("window", POINTER(c_int)), ("rope_theta", POINTER(c_float))]
+
+
+class ModernBertEncoderWeights(Structure):
+    _fields_ = [("tok_emb", c_void_p), ("emb_norm_w", c_void_p), ("emb_norm_b", c_void_p),
+                ("attn_norm_w", _PP), ("attn_norm_b", _PP),
+                ("Wqkv", _PP), ("Wqkv_b", _PP), ("Wo", _PP), ("Wo_b", _PP),
+                ("mlp_norm_w", _PP), ("mlp_norm_b", _PP),
+                ("Wi", _PP), ("Wi_b", _PP), ("mlp_Wo", _PP), ("mlp_Wo_b", _PP),
+                ("final_norm_w", c_void_p), ("final_norm_b", c_void_p)]
+
+
 _lib = None
 
 
@@ -113,6 +128,7 @@ def load_library() -> ctypes.CDLL:
     L.ac_ewc_penalty.argtypes = [POINTER(HeadParams), POINTER(HeadParams), POINTER(HeadParams), c_float, c_float,
                                  c_int, c_void_p, c_void_p]
     L.ac_encoder_create.argtypes = [POINTER(EncoderConfig), POINTER(EncoderWeights), POINTER(c_void_p)]
+    L.ac_encoder_create_modernbert.argtypes = [POINTER(ModernBertEncoderConfig), POINTER(ModernBertEncoderWeights), POINTER(c_void_p)]
     L.ac_encoder_destroy.argtypes = [c_void_p]
     L.ac_encoder_forward_cls.argtypes = [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p]
     L.ac_encoder_last_hidden.argtypes = [c_void_p, c_void_p, c_int64, c_void_p]
@@ -456,8 +472,42 @@ def distilbert_to_bert_state_dict(sd: dict, c):
     return out, dims
 
 
+def modernbert_dims(c) -> dict:
+    """HF ModernBertConfig -> the dimensions, per-layer key windows and rope thetas ac_encoder_create_modernbert takes.
+    Pure (no device work), so that an unsupported checkpoint is refused before anything is allocated."""
+    act = getattr(c, "hidden_activation", "gelu")
+    if act != "gelu":
+        raise AdaptiveB200Error(f"ModernBERT hidden_activation '{act}' is not implemented (exact-erf 'gelu' only)")
+    H, nh, I = int(c.hidden_size), int(c.num_attention_heads), int(c.intermediate_size)
+    if nh <= 0 or H % nh != 0 or H // nh != 64 or (getattr(c, "head_dim", None) or 64) != 64:
+        raise AdaptiveB200Error(f"ModernBERT head_dim must be 64 (hidden_size={H}, num_attention_heads={nh})")
+    if H % 128 != 0 or H > 1024:
+        raise AdaptiveB200Error(f"ModernBERT hidden_size={H} must be a multiple of 128 and <= 1024")
+    if I % 64 != 0:
+        raise AdaptiveB200Error(f"ModernBERT intermediate_size={I} must be a multiple of 64")
+    L = int(c.num_hidden_layers)
+    types = list(getattr(c, "layer_types", None) or [])
+    if len(types) != L:
+        raise AdaptiveB200Error(f"ModernBERT layer_types has {len(types)} entries for {L} layers")
+    rp = getattr(c, "rope_parameters", None) or {}
+    windows, thetas = [], []
+    for t in types:
+        if t not in ("full_attention", "sliding_attention"):
+            raise AdaptiveB200Error(f"ModernBERT layer type '{t}' is not implemented")
+        p = rp.get(t) if isinstance(rp, dict) else None
+        if not isinstance(p, dict) or "rope_theta" not in p:
+            raise AdaptiveB200Error(f"ModernBERT rope_parameters carry no rope_theta for '{t}'")
+        if p.get("rope_type", "default") != "default" or any(k not in ("rope_type", "rope_theta") for k in p):
+            raise AdaptiveB200Error(f"ModernBERT rope scaling {p} is not implemented (rope_type 'default' only)")
+        windows.append(int(c.sliding_window) if t == "sliding_attention" else 0)
+        thetas.append(float(p["rope_theta"]))
+    return dict(layers=L, hidden=H, heads=nh, intermediate=I, vocab=int(c.vocab_size), norm_eps=float(c.norm_eps),
+                windows=windows, thetas=thetas)
+
+
 class Encoder:
-    """Owner of an ac_encoder handle built from an HF BERT/RoBERTa state_dict (CUDA fp32 tensors)."""
+    """Owner of an ac_encoder handle built from an HF BERT/RoBERTa (or, through `modernbert`, ModernBERT) state_dict
+    (CUDA fp32 tensors)."""
 
     def __init__(self, sd: dict, *, arch: str, layers: int, hidden: int, heads: int, intermediate: int, vocab: int,
                  max_pos: int, type_vocab: int, ln_eps: float, pad_idx: int = 0, max_tokens: int = 65536,
@@ -503,10 +553,63 @@ class Encoder:
         del keep  # the handle holds its own packed copies
 
     @classmethod
+    def modernbert(cls, sd: dict, dims: dict, *, max_tokens: int = 65536, device="cuda", cls_only: bool = True):
+        """ac_encoder_create_modernbert over an HF ModernBertModel state_dict; dims = modernbert_dims(config)."""
+        L = load_library()
+        self = cls.__new__(cls)
+        self._L = L
+        self.hidden = dims["hidden"]
+        self.max_tokens = max_tokens
+        dev = torch.device(device)
+        n = dims["layers"]
+        keep = {}
+
+        def g(name):
+            t = sd.get(name)
+            if t is None:
+                return None
+            t = t.detach().to(device=dev, dtype=torch.float32).contiguous()
+            keep[name] = t
+            return t.data_ptr()
+
+        def arr(fmt, first=0):
+            a = (c_void_p * n)(*[(g(fmt.format(l)) if l >= first else None) for l in range(n)])
+            keep[fmt] = a
+            return ctypes.cast(a, _PP)
+
+        w = ModernBertEncoderWeights()
+        w.tok_emb = g("embeddings.tok_embeddings.weight")
+        w.emb_norm_w, w.emb_norm_b = g("embeddings.norm.weight"), g("embeddings.norm.bias")
+        p = "layers.{}."
+        w.attn_norm_w, w.attn_norm_b = arr(p + "attn_norm.weight", 1), arr(p + "attn_norm.bias", 1)
+        w.Wqkv, w.Wqkv_b = arr(p + "attn.Wqkv.weight"), arr(p + "attn.Wqkv.bias")
+        w.Wo, w.Wo_b = arr(p + "attn.Wo.weight"), arr(p + "attn.Wo.bias")
+        w.mlp_norm_w, w.mlp_norm_b = arr(p + "mlp_norm.weight"), arr(p + "mlp_norm.bias")
+        w.Wi, w.Wi_b = arr(p + "mlp.Wi.weight"), arr(p + "mlp.Wi.bias")
+        w.mlp_Wo, w.mlp_Wo_b = arr(p + "mlp.Wo.weight"), arr(p + "mlp.Wo.bias")
+        w.final_norm_w, w.final_norm_b = g("final_norm.weight"), g("final_norm.bias")
+        win = (c_int * n)(*dims["windows"])
+        th = (c_float * n)(*dims["thetas"])
+        cfg = ModernBertEncoderConfig(n, dims["hidden"], dims["heads"], dims["intermediate"], dims["vocab"], dims["norm_eps"],
+                                      AC_PREC_F16, max_tokens, 1 if cls_only else 0, win, th)
+        h = c_void_p()
+        with torch.cuda.device(dev):
+            check(L.ac_encoder_create_modernbert(ctypes.byref(cfg), ctypes.byref(w), ctypes.byref(h)),
+                  "ac_encoder_create_modernbert")
+        self.handle = h
+        del keep
+        return self
+
+    @classmethod
     def from_hf(cls, model, max_tokens: int = 65536, device="cuda", cls_only: bool = True):
-        """Build from an in-memory HF BertModel / RobertaModel / DistilBertModel (post-LN blocks, head_dim 64)."""
+        """Build from an in-memory HF BertModel / RobertaModel / DistilBertModel (post-LN blocks, head_dim 64) or
+        ModernBertModel (pre-LN, RoPE, GeGLU, sliding-window layers)."""
         c = model.config
         mt = getattr(c, "model_type", "bert")
+        if mt == "modernbert":
+            dims = modernbert_dims(c)
+            sd = {k: v for k, v in model.state_dict().items()}
+            return cls.modernbert(sd, dims, max_tokens=max_tokens, device=device, cls_only=cls_only)
         sd = {k: v for k, v in model.state_dict().items()}
         if mt == "distilbert":
             sd, dims = distilbert_to_bert_state_dict(sd, c)

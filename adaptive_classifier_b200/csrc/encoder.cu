@@ -545,9 +545,22 @@ constexpr int ATT_THREADS = 128;
 constexpr int ATT_SMEM = 48 * 1024 + 1024 /*align*/ + 64;
 constexpr int ATT_TMEM_COLS = 128;
 
+// bits lo..hi (clamped to 0..31) of a 32-key mask word: the keys of the word inside a query row's window
+__device__ __forceinline__ uint32_t window_bits(int lo, int hi) {
+    lo = max(lo, 0);
+    hi = min(hi, 31);
+    if (lo > hi) return 0u;
+    const uint32_t upto = (hi == 31) ? 0xffffffffu : ((1u << (hi + 1)) - 1u);
+    return upto & ~((1u << lo) - 1u);
+}
+
+// WIN (ModernBERT sliding layers, modeling_modernbert.py:262 / masking_utils.py:121-131): key k is visible to query q only
+// when |q - k| <= window (inclusive).  The window is folded into each query row's key bitmask, so a row whose window holds
+// no valid key ends with sum = 0 and writes zeros (never NaN / Inf).
+template <bool WIN>
 __global__ void __launch_bounds__(ATT_THREADS)
 attention_kernel(const __grid_constant__ CUtensorMap tmap_qk, const __grid_constant__ CUtensorMap tmap_vt,
-                 const int32_t *__restrict__ mask, int B, int S, int heads, int H, __half *__restrict__ ctx) {
+                 const int32_t *__restrict__ mask, int B, int S, int heads, int H, __half *__restrict__ ctx, int window) {
     extern __shared__ uint8_t smem_raw[];
     uint8_t *smem = reinterpret_cast<uint8_t *>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
     uint8_t *sQ = smem;                    // [128 rows x 128 B]
@@ -612,6 +625,10 @@ attention_kernel(const __grid_constant__ CUtensorMap tmap_qk, const __grid_const
         const int key = 32 * w4 + lane;
         const bool ok = (key < S) && (!mask || mask[row0 + key] != 0);
         kmask[w4] = __ballot_sync(0xffffffffu, ok);
+    }
+    if (WIN) {
+#pragma unroll
+        for (int w4 = 0; w4 < 4; ++w4) kmask[w4] &= window_bits(qrow - window - 32 * w4, qrow + window - 32 * w4);
     }
     const float scale_log2 = rsqrtf(64.f) * 1.44269504088896340736f;
     float mx = -CUDART_INF_F;
@@ -715,9 +732,12 @@ attention_kernel(const __grid_constant__ CUtensorMap tmap_qk, const __grid_const
 constexpr int ATTL_SMEM = 80 * 1024 + 1024 + 64;
 constexpr int ATTL_TMEM_COLS = 256;
 
+// WIN: the same per-row key window as attention_kernel; key blocks that lie entirely outside the window of every query of
+// this 128-query block are skipped (never loaded, never multiplied).
+template <bool WIN>
 __global__ void __launch_bounds__(ATT_THREADS)
 attention_long_kernel(const __grid_constant__ CUtensorMap tmap_qk, const __grid_constant__ CUtensorMap tmap_vt,
-                      const int32_t *__restrict__ mask, int B, int S, int heads, int H, __half *__restrict__ ctx) {
+                      const int32_t *__restrict__ mask, int B, int S, int heads, int H, __half *__restrict__ ctx, int window) {
     extern __shared__ uint8_t smem_raw[];
     uint8_t *smem = reinterpret_cast<uint8_t *>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
     uint8_t *sQ = smem;                    // [128 x 128 B]
@@ -734,6 +754,9 @@ attention_long_kernel(const __grid_constant__ CUtensorMap tmap_qk, const __grid_
     const int nkb = (S + 127) / 128;
     const int64_t row0 = static_cast<int64_t>(b) * S;
     const int vrow = (b * heads + h) * 64;
+    // key blocks [jlo, jend) can hold a visible key of this query block
+    const int jlo = WIN ? max(qb * 128 - window, 0) / 128 : 0;
+    const int jend = WIN ? min((min(qb * 128 + 127, S - 1) + window) / 128 + 1, nkb) : nkb;
 
     if (tid == 0) {
         tma_prefetch_desc(&tmap_qk);
@@ -762,10 +785,10 @@ attention_long_kernel(const __grid_constant__ CUtensorMap tmap_qk, const __grid_
     float mx = -CUDART_INF_F, sum = 0.f;
 
     for (int pass = 0; pass < 2; ++pass) {
-        for (int j = 0; j < nkb; ++j) {
+        for (int j = jlo; j < jend; ++j) {
             const int key0 = j * 128;
             if (tid == 0) {
-                const bool first = (pass == 0 && j == 0);
+                const bool first = (pass == 0 && j == jlo);
                 const uint32_t bytes = (first ? 16 * 1024 : 0) + 16 * 1024 + (pass == 1 ? 16 * 1024 : 0);
                 mbar_arrive_expect_tx(bar_load, bytes);
                 if (first) tma_load_2d(sQ, &tmap_qk, bar_load, h * 64, static_cast<int>(row0) + qb * 128);
@@ -795,6 +818,13 @@ attention_long_kernel(const __grid_constant__ CUtensorMap tmap_qk, const __grid_
                 const int key = key0 + 32 * w4 + lane;
                 const bool ok = (key < S) && (!mask || mask[row0 + key] != 0);
                 kmask[w4] = __ballot_sync(0xffffffffu, ok);
+            }
+            if (WIN) {
+#pragma unroll
+                for (int w4 = 0; w4 < 4; ++w4) {
+                    const int k0 = key0 + 32 * w4;
+                    kmask[w4] &= window_bits(qglob - window - k0, qglob + window - k0);
+                }
             }
             if (pass == 0) {
 #pragma unroll
@@ -849,7 +879,7 @@ attention_long_kernel(const __grid_constant__ CUtensorMap tmap_qk, const __grid_
                         const uint64_t bd = umma_desc_sw128(smem_u32(sVt + slab * 8192));
 #pragma unroll
                         for (int k = 0; k < 4; ++k)
-                            umma_f16(tmem_base + 128, a + 2 * k, bd + 2 * k, idesc_o, (j | slab | k) != 0);
+                            umma_f16(tmem_base + 128, a + 2 * k, bd + 2 * k, idesc_o, ((WIN ? j - jlo : j) | slab | k) != 0);
                     }
                     tc_commit(bar_o);
                 }
@@ -908,6 +938,176 @@ __global__ void gather_cls_ln_kernel(const __half *__restrict__ ctx, const float
     ln_row(x, nv, H, g, b, eps, lane, x_cls + dst, nullptr);
 }
 
+// ================================================================================================
+// ModernBERT (HF modeling_modernbert.py): pre-LN blocks, RoPE attention with per-layer windows, GeGLU FFN
+// ================================================================================================
+
+// modeling_modernbert.py:52-71: LayerNorm(tok_embeddings[ids]); no position or token-type rows
+__global__ void embed_norm_kernel(const int32_t *__restrict__ ids, const float *__restrict__ tok, const float *__restrict__ w,
+                                  const float *__restrict__ b, float eps, int rows, int H, int vocab, float *__restrict__ out_full,
+                                  __half *__restrict__ out_half) {
+    const int row = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    const int lane = threadIdx.x & 31;
+    if (row >= rows) return;
+    const int id = min(max(ids[row], 0), vocab - 1);
+    const int nv = H / 128;
+    float4 x[LN_MAXV];
+#pragma unroll
+    for (int i = 0; i < LN_MAXV; ++i)
+        if (i < nv) x[i] = __ldg(reinterpret_cast<const float4 *>(tok + static_cast<int64_t>(id) * H + (lane + 32 * i) * 4));
+    ln_row(x, nv, H, w, b, eps, lane, out_full + static_cast<int64_t>(row) * H, out_half + static_cast<int64_t>(row) * H);
+}
+
+// 32 fp32 values of one accumulator row -> fp16 Y[row_base + lane, col0 .. col0 + 32) through the warp's staging tile
+// (the store pattern of EpiLinear's fp16 path: 8 rows x 4 x 16 B per pass)
+__device__ __forceinline__ void store_row32_half(const float (&y)[32], uint8_t *stage, int lane, int row_base, int col0, int M,
+                                                 int N, int ldy, __half *Y) {
+    uint4 *srow = reinterpret_cast<uint4 *>(stage + lane * GEMM_EPI_STAGE_ROW_BYTES);
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+        uint4 pk;
+        __half2 h0 = __floats2half2_rn(y[8 * j], y[8 * j + 1]), h1 = __floats2half2_rn(y[8 * j + 2], y[8 * j + 3]);
+        __half2 h2 = __floats2half2_rn(y[8 * j + 4], y[8 * j + 5]), h3 = __floats2half2_rn(y[8 * j + 6], y[8 * j + 7]);
+        pk.x = *reinterpret_cast<uint32_t *>(&h0); pk.y = *reinterpret_cast<uint32_t *>(&h1);
+        pk.z = *reinterpret_cast<uint32_t *>(&h2); pk.w = *reinterpret_cast<uint32_t *>(&h3);
+        srow[j] = pk;
+    }
+    __syncwarp();
+    const int r8 = lane >> 2, c = lane & 3;
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+        const int rr = r8 + 8 * i;
+        const int grow = row_base + rr;
+        const int col = col0 + 8 * c;
+        if (grow < M && col + 8 <= N) {
+            const uint4 pk = *reinterpret_cast<const uint4 *>(stage + rr * GEMM_EPI_STAGE_ROW_BYTES + 16 * c);
+            *reinterpret_cast<uint4 *>(Y + static_cast<int64_t>(grow) * ldy + col) = pk;
+        }
+    }
+    __syncwarp();
+}
+
+// fused Wqkv epilogue (modeling_modernbert.py:285-296): acc + bias, RoPE on the q and k thirds in fp32 before the fp16
+// rounding, V third written transposed as EpiLinear's VT path does.  One epilogue warp drains 128 columns (two whole heads)
+// in 32-column chunks, so the thread holding head columns d = 0..31 of its row receives d = 32..63 in the next chunk: the
+// first half waits in registers, the second chunk rotates both (rotate_half pairs d with d + 32) and stores 64 columns.
+//   q'[d]      = q[d] cos - q[d + 32] sin        q'[d + 32] = q[d + 32] cos + q[d] sin       (cos, sin of angle pos * f_d)
+// cs: [512 positions][32] (cos, sin) for this layer's theta, position = row % S (position_ids = arange(S)).
+struct EpiQKVRope {
+    const float *__restrict__ bias;       // [3H]
+    __half *qk;                           // [M, 2H] rotated q | k
+    __half *vT;                           // [(b, feature), S_pad] V^T
+    const float2 *__restrict__ cs;        // [512, 32]
+    int M, H, S, S_pad;
+
+    static constexpr int kUnrollChunks = 4;
+    static constexpr int kPrefetchDist = 1;
+    struct State {
+        float lo[32];                     // head columns 0..31 (acc + bias) of the chunk drained before
+    };
+    __device__ __forceinline__ void begin_cta(State &, int, int) const {}
+    __device__ __forceinline__ void end_cta(State &, int, int) const {}
+    __device__ __forceinline__ void prefetch(State &, const GemmTileInfo &, int, int, int, int) const {}
+
+    __device__ __forceinline__ void tile(State &st, const GemmTileInfo &ti, int row, int col0, const float (&v)[32],
+                                         uint8_t *stage, int lane, int, uint32_t) const {
+        const int row_base = ti.m0 + ((threadIdx.x >> 5) & 3) * 32;
+        if (row_base >= M || col0 >= 3 * H) return;                        // warp-uniform
+        if (col0 >= 2 * H) {
+            if (row < M) {
+                const int b = row / S, key = row - b * S;
+                __half *dst = vT + (static_cast<int64_t>(b) * H + (col0 - 2 * H)) * S_pad + key;
+#pragma unroll
+                for (int j = 0; j < 32; j += 4) {
+                    const float4 b4 = __ldg(reinterpret_cast<const float4 *>(bias + col0 + j));
+                    dst[static_cast<int64_t>(j) * S_pad] = __float2half_rn(v[j] + b4.x);
+                    dst[static_cast<int64_t>(j + 1) * S_pad] = __float2half_rn(v[j + 1] + b4.y);
+                    dst[static_cast<int64_t>(j + 2) * S_pad] = __float2half_rn(v[j + 2] + b4.z);
+                    dst[static_cast<int64_t>(j + 3) * S_pad] = __float2half_rn(v[j + 3] + b4.w);
+                }
+            }
+            return;
+        }
+        if ((col0 & 32) == 0) {                                              // head columns 0..31: keep for the next chunk
+#pragma unroll
+            for (int j = 0; j < 32; j += 4) {
+                const float4 b4 = __ldg(reinterpret_cast<const float4 *>(bias + col0 + j));
+                st.lo[j] = v[j] + b4.x; st.lo[j + 1] = v[j + 1] + b4.y;
+                st.lo[j + 2] = v[j + 2] + b4.z; st.lo[j + 3] = v[j + 3] + b4.w;
+            }
+            return;
+        }
+        const int pos = (row < M) ? row % S : 0;
+        const float4 *cs4 = reinterpret_cast<const float4 *>(cs + pos * 32);   // (cos, sin) of d, d + 1
+        // both halves in one pass: the rotated first half overwrites st.lo, the second half goes to hi (peak 64 live values)
+        float hi[32];
+#pragma unroll
+        for (int j = 0; j < 32; j += 2) {
+            const float4 t = __ldg(cs4 + (j >> 1));
+            const float2 b2 = __ldg(reinterpret_cast<const float2 *>(bias + col0 + j));
+            const float h0 = v[j] + b2.x, h1 = v[j + 1] + b2.y;
+            const float l0 = st.lo[j], l1 = st.lo[j + 1];
+            st.lo[j] = fmaf(l0, t.x, -h0 * t.y);
+            st.lo[j + 1] = fmaf(l1, t.z, -h1 * t.w);
+            hi[j] = fmaf(h0, t.x, l0 * t.y);
+            hi[j + 1] = fmaf(h1, t.z, l1 * t.w);
+        }
+        store_row32_half(st.lo, stage, lane, row_base, col0 - 32, M, 2 * H, 2 * H, qk);
+        store_row32_half(hi, stage, lane, row_base, col0, M, 2 * H, 2 * H, qk);
+    }
+};
+
+// GeGLU FFN1 epilogue (modeling_modernbert.py:88-91): Wi is packed at create time so that accumulator chunk q (32 columns)
+// holds input columns 16q .. 16q+15 followed by the matching gate columns I + 16q ..; the thread of a row writes
+// gelu_erf(input + b) * (gate + b') as 16 fp16 values (one 32-byte sector) at output columns 16q .. 16q+15 of Y[M, I].
+// Chunks at or past N = 2I are skipped (the last 256-column tile of ModernBERT-large's 2I = 5248 is half empty).
+struct EpiGeGLU {
+    const float *__restrict__ bias;       // [2I] in packed order
+    __half *Y;                            // [M, I]
+    int M, N, I;
+
+    static constexpr int kUnrollChunks = 4;
+    static constexpr int kPrefetchDist = 1;
+    struct State {};
+    __device__ __forceinline__ void begin_cta(State &, int, int) const {}
+    __device__ __forceinline__ void end_cta(State &, int, int) const {}
+    __device__ __forceinline__ void prefetch(State &, const GemmTileInfo &, int, int, int, int) const {}
+
+    __device__ __forceinline__ void tile(State &, const GemmTileInfo &, int row, int col0, const float (&v)[32], uint8_t *,
+                                         int, int, uint32_t) const {
+        if (row >= M || col0 >= N) return;
+        uint32_t pk[8];
+#pragma unroll
+        for (int j = 0; j < 16; j += 4) {
+            const float4 ba = __ldg(reinterpret_cast<const float4 *>(bias + col0 + j));
+            const float4 bg = __ldg(reinterpret_cast<const float4 *>(bias + col0 + 16 + j));
+            const __half2 h0 = __floats2half2_rn(gelu_erf(v[j] + ba.x) * (v[16 + j] + bg.x),
+                                                 gelu_erf(v[j + 1] + ba.y) * (v[17 + j] + bg.y));
+            const __half2 h1 = __floats2half2_rn(gelu_erf(v[j + 2] + ba.z) * (v[18 + j] + bg.z),
+                                                 gelu_erf(v[j + 3] + ba.w) * (v[19 + j] + bg.w));
+            pk[j >> 1] = *reinterpret_cast<const uint32_t *>(&h0);
+            pk[(j >> 1) + 1] = *reinterpret_cast<const uint32_t *>(&h1);
+        }
+        uint4 *dst = reinterpret_cast<uint4 *>(Y + static_cast<int64_t>(row) * I + (col0 >> 1));
+        dst[0] = make_uint4(pk[0], pk[1], pk[2], pk[3]);
+        dst[1] = make_uint4(pk[4], pk[5], pk[6], pk[7]);
+    }
+};
+
+// Wi [2I, H] (fp32, HF rows: input 0..I-1, gate I..2I-1) -> fp16 rows in the chunk order EpiGeGLU reads, bias likewise
+// (NULL bias = zeros).  Packed row p = 32 q + j: input row 16 q + j (j < 16) or gate row I + 16 q + j - 16.
+__global__ void pack_geglu_kernel(const float *__restrict__ W, const float *__restrict__ bias, int I, int K, __half *__restrict__ Wp,
+                                  float *__restrict__ bp) {
+    const int p = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    const int lane = threadIdx.x & 31;
+    if (p >= 2 * I) return;
+    const int q = p >> 5, j = p & 31;
+    const int src = (j < 16) ? 16 * q + j : I + 16 * q + (j - 16);
+    for (int k = lane; k < K; k += 32)
+        Wp[static_cast<int64_t>(p) * K + k] = __float2half_rn(W[static_cast<int64_t>(src) * K + k]);
+    if (lane == 0) bp[p] = bias ? bias[src] : 0.f;
+}
+
 }  // namespace ac
 
 // ================================================================================================
@@ -947,6 +1147,12 @@ struct ac_encoder {
     int last_B = 0, last_S = 0;
     bool last_cls_only = false;
     const float *last_hidden = nullptr;   // where the previous full forward left the last hidden state
+    // ModernBERT (AC_ARCH_MODERNBERT): word = tok_embeddings, emb_ln_* = embeddings.norm; per layer wqkv_d = plain fp16 Wqkv,
+    // wo / bo = attn.Wo, w1_d = Wi packed for EpiGeGLU, w2 / b2 = mlp.Wo (their tensor maps as above), and:
+    std::vector<float *> bqkv, bi, attn_nw, attn_nb, mlp_nw, mlp_nb;   // biases (zeros when absent), LayerNorms (attn_* unused in layer 0)
+    std::vector<float2 *> rope;           // per layer [512, 32] (cos, sin) of its theta
+    std::vector<int> window;              // per layer key window, 0 = global
+    float *final_nw = nullptr, *final_nb = nullptr;
 };
 
 static int launch_cls_normalize(const float *x, int B, int S, int H, float *out, cudaStream_t s) {
@@ -957,7 +1163,7 @@ static int launch_cls_normalize(const float *x, int B, int S, int H, float *out,
 }
 
 // softmax(Q K^T / 8 + mask) V out of e->qk / e->vT into e->ctx
-static int launch_attention(ac_encoder *e, const int32_t *mask, int B, int S, cudaStream_t s) {
+static int launch_attention(ac_encoder *e, const int32_t *mask, int B, int S, cudaStream_t s, int window = 0) {
     const ac_encoder_config &c = e->cfg;
     const int H = c.hidden;
     // per-device: the attribute is a property of the (function, device) pair
@@ -965,17 +1171,28 @@ static int launch_attention(ac_encoder *e, const int32_t *mask, int B, int S, cu
     int dev = 0;
     AC_CUDA(cudaGetDevice(&dev));
     if (dev < 0 || dev >= 64 || !att_attr[dev]) {
-        AC_CUDA(cudaFuncSetAttribute(attention_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, ATT_SMEM));
-        AC_CUDA(cudaFuncSetAttribute(attention_long_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, ATTL_SMEM));
+        AC_CUDA(cudaFuncSetAttribute(attention_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, ATT_SMEM));
+        AC_CUDA(cudaFuncSetAttribute(attention_long_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, ATTL_SMEM));
+        AC_CUDA(cudaFuncSetAttribute(attention_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, ATT_SMEM));
+        AC_CUDA(cudaFuncSetAttribute(attention_long_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, ATTL_SMEM));
         if (dev >= 0 && dev < 64) att_attr[dev] = true;
     }
     // algorithmic flops of softmax(QK^T)V at the true sequence length (the 128-wide tile does more)
+    // a window that covers the whole sequence is global attention
+    const bool win = window > 0 && window < S - 1;
     const int slot = prof_begin(PROF_ATTENTION, 4.0 * B * c.heads * static_cast<double>(S) * S * 64, 0.0, s);
-    if (S <= 128)
-        attention_kernel<<<B * c.heads, ATT_THREADS, ATT_SMEM, s>>>(e->m_qk_att, e->m_vt_att, mask, B, S, c.heads, H, e->ctx);
+    const dim3 grid_long(B * c.heads, (S + 127) / 128);
+    if (S <= 128 && win)
+        attention_kernel<true><<<B * c.heads, ATT_THREADS, ATT_SMEM, s>>>(e->m_qk_att, e->m_vt_att, mask, B, S, c.heads, H, e->ctx,
+                                                                          window);
+    else if (S <= 128)
+        attention_kernel<false><<<B * c.heads, ATT_THREADS, ATT_SMEM, s>>>(e->m_qk_att, e->m_vt_att, mask, B, S, c.heads, H, e->ctx, 0);
+    else if (win)
+        attention_long_kernel<true><<<grid_long, ATT_THREADS, ATTL_SMEM, s>>>(e->m_qk_att, e->m_vt_att, mask, B, S, c.heads, H,
+                                                                               e->ctx, window);
     else
-        attention_long_kernel<<<dim3(B * c.heads, (S + 127) / 128), ATT_THREADS, ATTL_SMEM, s>>>(e->m_qk_att, e->m_vt_att, mask, B, S,
-                                                                                                c.heads, H, e->ctx);
+        attention_long_kernel<false><<<grid_long, ATT_THREADS, ATTL_SMEM, s>>>(e->m_qk_att, e->m_vt_att, mask, B, S, c.heads, H,
+                                                                                e->ctx, 0);
     prof_end(slot, s);
     AC_LAUNCH_CHECK();
     return AC_OK;
@@ -1009,6 +1226,56 @@ extern "C" int ac_encoder_destroy(ac_encoder *enc) {
     if (!enc) return AC_OK;
     for (void *p : enc->allocs) cudaFree(p);
     delete enc;
+    return AC_OK;
+}
+
+// activation workspace, row statistics and the A-operand tensor maps of an encoder sized by e->cfg (both architectures)
+static int alloc_workspace(ac_encoder *e) {
+    const int H = e->cfg.hidden, I = e->cfg.intermediate;
+    const size_t T = e->T;
+    int rc;
+#define WS(x) do { rc = (x); if (rc) return rc; } while (0)
+    WS(dev_alloc(e, &e->stats_a, T));
+    WS(dev_alloc(e, &e->stats_b, T));
+    WS(dev_alloc(e, &e->stats_id, T));
+    WS(dev_alloc(e, &e->parts, static_cast<size_t>(H / 128) * T));
+    WS(dev_alloc(e, &e->ones, H));
+    WS(dev_alloc(e, &e->zeros, H));
+    fill_stats_identity_kernel<<<static_cast<unsigned>((T + 255) / 256), 256>>>(e->stats_id, static_cast<int64_t>(T));
+    fill_value_kernel<<<(H + 255) / 256, 256>>>(e->ones, H, 1.f);
+    fill_value_kernel<<<(H + 255) / 256, 256>>>(e->zeros, H, 0.f);
+    WS(check_cuda(cudaGetLastError(), "deferred-LayerNorm constants"));
+    e->vt_elems = 2 * T * H;     // (b, h, d) rows x S_pad keys, S_pad = roundup(S, 8) <= 2*S for S >= 8
+    WS(dev_alloc(e, &e->x, T * H));
+    WS(dev_alloc(e, &e->tmp, T * H));
+    WS(dev_alloc(e, &e->xh, T * H));
+    WS(dev_alloc(e, &e->qk, T * 2 * H));
+    WS(dev_alloc(e, &e->vT, e->vt_elems));
+    WS(dev_alloc(e, &e->ctx, T * H));
+    WS(dev_alloc(e, &e->ffn, T * I));
+    e->Bc = T < 16384 ? T : 16384;
+    WS(dev_alloc(e, &e->x_cls, e->Bc * H));
+    WS(dev_alloc(e, &e->tmp_cls, e->Bc * H));
+    WS(dev_alloc(e, &e->xh_cls, e->Bc * H));
+    WS(dev_alloc(e, &e->ctx_cls, e->Bc * H));
+    WS(dev_alloc(e, &e->ffn_cls, e->Bc * I));
+    WS(check_cuda(cudaMemset(e->xh_cls, 0, e->Bc * H * sizeof(__half)), "memset xh_cls"));
+    WS(check_cuda(cudaMemset(e->ctx_cls, 0, e->Bc * H * sizeof(__half)), "memset ctx_cls"));
+    WS(check_cuda(cudaMemset(e->ffn_cls, 0, e->Bc * I * sizeof(__half)), "memset ffn_cls"));
+    WS(check_cuda(cudaMemset(e->qk, 0, T * 2 * H * sizeof(__half)), "memset qk"));
+    WS(check_cuda(cudaMemset(e->vT, 0, e->vt_elems * sizeof(__half)), "memset vT"));
+    WS(check_cuda(cudaMemset(e->xh, 0, T * H * sizeof(__half)), "memset xh"));
+    WS(check_cuda(cudaMemset(e->ctx, 0, T * H * sizeof(__half)), "memset ctx"));
+    WS(check_cuda(cudaMemset(e->ffn, 0, T * I * sizeof(__half)), "memset ffn"));
+    // TMA descriptors (fp16: 64 elements = 128 bytes per box row)
+    WS(make_tmap_2d(&e->m_xh, e->xh, 2, T, H, static_cast<uint64_t>(H) * 2, GEMM_BLOCK_M, 64));
+    WS(make_tmap_2d(&e->m_ctx, e->ctx, 2, T, H, static_cast<uint64_t>(H) * 2, GEMM_BLOCK_M, 64));
+    WS(make_tmap_2d(&e->m_ffn, e->ffn, 2, T, I, static_cast<uint64_t>(I) * 2, GEMM_BLOCK_M, 64));
+    WS(make_tmap_2d(&e->m_qk_att, e->qk, 2, T, 2 * H, static_cast<uint64_t>(2 * H) * 2, 128, 64));
+    WS(make_tmap_2d(&e->m_xh_cls, e->xh_cls, 2, e->Bc, H, static_cast<uint64_t>(H) * 2, GEMM_BLOCK_M, 64));
+    WS(make_tmap_2d(&e->m_ctx_cls, e->ctx_cls, 2, e->Bc, H, static_cast<uint64_t>(H) * 2, GEMM_BLOCK_M, 64));
+    WS(make_tmap_2d(&e->m_ffn_cls, e->ffn_cls, 2, e->Bc, I, static_cast<uint64_t>(I) * 2, GEMM_BLOCK_M, 64));
+#undef WS
     return AC_OK;
 }
 
@@ -1071,46 +1338,7 @@ extern "C" int ac_encoder_create(const ac_encoder_config *cfg, const ac_encoder_
         TRY(pack_f16(e, &e->w1_last, w->ff1_w[L - 1], static_cast<size_t>(I) * H));
         TRY(pack_f32(e, &e->b1_last, w->ff1_b[L - 1], I));
     }
-    TRY(dev_alloc(e, &e->stats_a, T));
-    TRY(dev_alloc(e, &e->stats_b, T));
-    TRY(dev_alloc(e, &e->stats_id, T));
-    TRY(dev_alloc(e, &e->parts, static_cast<size_t>(H / 128) * T));
-    TRY(dev_alloc(e, &e->ones, H));
-    TRY(dev_alloc(e, &e->zeros, H));
-    fill_stats_identity_kernel<<<static_cast<unsigned>((T + 255) / 256), 256>>>(e->stats_id, static_cast<int64_t>(T));
-    fill_value_kernel<<<(H + 255) / 256, 256>>>(e->ones, H, 1.f);
-    fill_value_kernel<<<(H + 255) / 256, 256>>>(e->zeros, H, 0.f);
-    TRY(check_cuda(cudaGetLastError(), "deferred-LayerNorm constants"));
-    e->vt_elems = 2 * T * H;     // (b, h, d) rows x S_pad keys, S_pad = roundup(S, 8) <= 2*S for S >= 8
-    TRY(dev_alloc(e, &e->x, T * H));
-    TRY(dev_alloc(e, &e->tmp, T * H));
-    TRY(dev_alloc(e, &e->xh, T * H));
-    TRY(dev_alloc(e, &e->qk, T * 2 * H));
-    TRY(dev_alloc(e, &e->vT, e->vt_elems));
-    TRY(dev_alloc(e, &e->ctx, T * H));
-    TRY(dev_alloc(e, &e->ffn, T * I));
-    e->Bc = T < 16384 ? T : 16384;
-    TRY(dev_alloc(e, &e->x_cls, e->Bc * H));
-    TRY(dev_alloc(e, &e->tmp_cls, e->Bc * H));
-    TRY(dev_alloc(e, &e->xh_cls, e->Bc * H));
-    TRY(dev_alloc(e, &e->ctx_cls, e->Bc * H));
-    TRY(dev_alloc(e, &e->ffn_cls, e->Bc * I));
-    TRY(check_cuda(cudaMemset(e->xh_cls, 0, e->Bc * H * sizeof(__half)), "memset xh_cls"));
-    TRY(check_cuda(cudaMemset(e->ctx_cls, 0, e->Bc * H * sizeof(__half)), "memset ctx_cls"));
-    TRY(check_cuda(cudaMemset(e->ffn_cls, 0, e->Bc * I * sizeof(__half)), "memset ffn_cls"));
-    TRY(check_cuda(cudaMemset(e->qk, 0, T * 2 * H * sizeof(__half)), "memset qk"));
-    TRY(check_cuda(cudaMemset(e->vT, 0, e->vt_elems * sizeof(__half)), "memset vT"));
-    TRY(check_cuda(cudaMemset(e->xh, 0, T * H * sizeof(__half)), "memset xh"));
-    TRY(check_cuda(cudaMemset(e->ctx, 0, T * H * sizeof(__half)), "memset ctx"));
-    TRY(check_cuda(cudaMemset(e->ffn, 0, T * I * sizeof(__half)), "memset ffn"));
-    // TMA descriptors (fp16: 64 elements = 128 bytes per box row)
-    TRY(make_tmap_2d(&e->m_xh, e->xh, 2, T, H, static_cast<uint64_t>(H) * 2, GEMM_BLOCK_M, 64));
-    TRY(make_tmap_2d(&e->m_ctx, e->ctx, 2, T, H, static_cast<uint64_t>(H) * 2, GEMM_BLOCK_M, 64));
-    TRY(make_tmap_2d(&e->m_ffn, e->ffn, 2, T, I, static_cast<uint64_t>(I) * 2, GEMM_BLOCK_M, 64));
-    TRY(make_tmap_2d(&e->m_qk_att, e->qk, 2, T, 2 * H, static_cast<uint64_t>(2 * H) * 2, 128, 64));
-    TRY(make_tmap_2d(&e->m_xh_cls, e->xh_cls, 2, e->Bc, H, static_cast<uint64_t>(H) * 2, GEMM_BLOCK_M, 64));
-    TRY(make_tmap_2d(&e->m_ctx_cls, e->ctx_cls, 2, e->Bc, H, static_cast<uint64_t>(H) * 2, GEMM_BLOCK_M, 64));
-    TRY(make_tmap_2d(&e->m_ffn_cls, e->ffn_cls, 2, e->Bc, I, static_cast<uint64_t>(I) * 2, GEMM_BLOCK_M, 64));
+    TRY(alloc_workspace(e));
     e->p_wqkv_d.resize(L); e->p_wo.resize(L); e->p_w1_d.resize(L); e->p_w2.resize(L);
     for (int l = 0; l < L; ++l) {
         TRY(make_tmap_2d(&e->p_wqkv_d[l], e->wqkv_d[l], 2, 3 * H, H, static_cast<uint64_t>(H) * 2, GEMM2_B_ROWS, 64));
@@ -1120,6 +1348,103 @@ extern "C" int ac_encoder_create(const ac_encoder_config *cfg, const ac_encoder_
     }
     if (cfg->cls_only) TRY(make_tmap_2d(&e->p_w1_last, e->w1_last, 2, I, H, static_cast<uint64_t>(H) * 2, GEMM2_B_ROWS, 64));
     TRY(check_cuda(cudaDeviceSynchronize(), "encoder_create sync"));
+#undef TRY
+    *out = e;
+    return AC_OK;
+}
+
+// fp32 copy of src, or n zeros when src is NULL (absent biases of ModernBERT's norm_bias / attention_bias / mlp_bias = False)
+static int pack_f32_or_zero(ac_encoder *e, float **dst, const float *src, size_t n) {
+    if (src) return pack_f32(e, dst, src, n);
+    int rc = dev_alloc(e, dst, n);
+    if (rc) return rc;
+    AC_CUDA(cudaMemset(*dst, 0, n * sizeof(float)));
+    return AC_OK;
+}
+
+constexpr int ROPE_MAX_POS = 512;
+
+extern "C" int ac_encoder_create_modernbert(const ac_modernbert_config *cfg, const ac_modernbert_weights *w, ac_encoder **out) {
+    AC_REQUIRE(cfg && w && out, "ac_encoder_create_modernbert: null argument");
+    AC_REQUIRE(cfg->precision == AC_PREC_F16, "ac_encoder_create_modernbert: only AC_PREC_F16 is implemented");
+    AC_REQUIRE(cfg->hidden % 128 == 0 && cfg->hidden > 0 && cfg->hidden <= 1024,
+               "ac_encoder_create_modernbert: hidden=%d must be a multiple of 128, <= 1024", cfg->hidden);
+    AC_REQUIRE(cfg->heads > 0 && cfg->hidden % cfg->heads == 0 && cfg->hidden / cfg->heads == 64,
+               "ac_encoder_create_modernbert: head_dim must be 64 (hidden=%d heads=%d)", cfg->hidden, cfg->heads);
+    AC_REQUIRE(cfg->intermediate > 0 && cfg->intermediate % 64 == 0,
+               "ac_encoder_create_modernbert: intermediate=%d must be a multiple of 64", cfg->intermediate);
+    AC_REQUIRE(cfg->layers > 0 && cfg->max_tokens > 0 && cfg->vocab > 0, "ac_encoder_create_modernbert: bad dims");
+    AC_REQUIRE(cfg->window && cfg->rope_theta, "ac_encoder_create_modernbert: window and rope_theta arrays are required");
+    for (int l = 0; l < cfg->layers; ++l)
+        AC_REQUIRE(cfg->window[l] >= 0 && cfg->rope_theta[l] > 0.f, "ac_encoder_create_modernbert: layer %d: window=%d theta=%g",
+                   l, cfg->window[l], static_cast<double>(cfg->rope_theta[l]));
+    AC_REQUIRE(w->tok_emb && w->emb_norm_w && w->final_norm_w && w->Wqkv && w->Wo && w->mlp_norm_w && w->Wi && w->mlp_Wo &&
+                   (cfg->layers == 1 || w->attn_norm_w),
+               "ac_encoder_create_modernbert: missing weight");
+    int rc = ac_device_check();
+    if (rc) return rc;
+    ac_encoder *e = new ac_encoder();
+    ac_encoder_config &c = e->cfg;
+    c.arch = AC_ARCH_MODERNBERT;
+    c.layers = cfg->layers; c.hidden = cfg->hidden; c.heads = cfg->heads; c.intermediate = cfg->intermediate;
+    c.vocab = cfg->vocab; c.max_pos = ROPE_MAX_POS; c.type_vocab = 1; c.pad_idx = 0;
+    c.ln_eps = cfg->norm_eps; c.precision = cfg->precision; c.max_tokens = cfg->max_tokens; c.cls_only = cfg->cls_only;
+    const int H = c.hidden, I = c.intermediate, L = c.layers;
+    e->T = static_cast<size_t>((cfg->max_tokens + 127) / 128 * 128);
+    auto at = [](const float *const *a, int l) -> const float * { return a ? a[l] : nullptr; };
+#define TRY(x) do { rc = (x); if (rc) { ac_encoder_destroy(e); return rc; } } while (0)
+    TRY(pack_f32(e, &e->word, w->tok_emb, static_cast<size_t>(c.vocab) * H));
+    TRY(pack_f32(e, &e->emb_ln_w, w->emb_norm_w, H));
+    TRY(pack_f32_or_zero(e, &e->emb_ln_b, w->emb_norm_b, H));
+    TRY(pack_f32(e, &e->final_nw, w->final_norm_w, H));
+    TRY(pack_f32_or_zero(e, &e->final_nb, w->final_norm_b, H));
+    e->wqkv_d.assign(L, nullptr); e->wo.assign(L, nullptr); e->w1_d.assign(L, nullptr); e->w2.assign(L, nullptr);
+    e->bqkv.assign(L, nullptr); e->bo.assign(L, nullptr); e->bi.assign(L, nullptr); e->b2.assign(L, nullptr);
+    e->attn_nw.assign(L, nullptr); e->attn_nb.assign(L, nullptr); e->mlp_nw.assign(L, nullptr); e->mlp_nb.assign(L, nullptr);
+    e->rope.assign(L, nullptr);
+    e->window.assign(cfg->window, cfg->window + L);
+    const size_t HH = static_cast<size_t>(H) * H;
+    std::vector<float2> cs(static_cast<size_t>(ROPE_MAX_POS) * 32);
+    for (int l = 0; l < L; ++l) {
+        if (l > 0) {
+            TRY(pack_f32(e, &e->attn_nw[l], w->attn_norm_w[l], H));
+            TRY(pack_f32_or_zero(e, &e->attn_nb[l], at(w->attn_norm_b, l), H));
+        }
+        TRY(pack_f16(e, &e->wqkv_d[l], w->Wqkv[l], 3 * HH));
+        TRY(pack_f32_or_zero(e, &e->bqkv[l], at(w->Wqkv_b, l), 3 * static_cast<size_t>(H)));
+        TRY(pack_f16(e, &e->wo[l], w->Wo[l], HH));
+        TRY(pack_f32_or_zero(e, &e->bo[l], at(w->Wo_b, l), H));
+        TRY(pack_f32(e, &e->mlp_nw[l], w->mlp_norm_w[l], H));
+        TRY(pack_f32_or_zero(e, &e->mlp_nb[l], at(w->mlp_norm_b, l), H));
+        TRY(dev_alloc(e, &e->w1_d[l], 2 * static_cast<size_t>(I) * H));
+        TRY(dev_alloc(e, &e->bi[l], 2 * static_cast<size_t>(I)));
+        pack_geglu_kernel<<<(2 * I + 7) / 8, 256>>>(w->Wi[l], at(w->Wi_b, l), I, H, e->w1_d[l], e->bi[l]);
+        TRY(check_cuda(cudaGetLastError(), "pack_geglu_kernel"));
+        TRY(pack_f16(e, &e->w2[l], w->mlp_Wo[l], static_cast<size_t>(H) * I));
+        TRY(pack_f32_or_zero(e, &e->b2[l], at(w->mlp_Wo_b, l), H));
+        // RoPE table of this layer's theta, as HF computes it (modeling_modernbert.py:121-154): inv_freq = 1 / theta^(2i/64)
+        // and angle = position * inv_freq in fp32, cos / sin of the fp32 angle
+        const float theta = cfg->rope_theta[l];
+        for (int i = 0; i < 32; ++i) {
+            const float inv = 1.0f / powf(theta, static_cast<float>(2 * i) / 64.f);
+            for (int pos = 0; pos < ROPE_MAX_POS; ++pos) {
+                const float ang = static_cast<float>(pos) * inv;
+                cs[static_cast<size_t>(pos) * 32 + i] = make_float2(static_cast<float>(cos(static_cast<double>(ang))),
+                                                                    static_cast<float>(sin(static_cast<double>(ang))));
+            }
+        }
+        TRY(dev_alloc(e, &e->rope[l], cs.size()));
+        TRY(check_cuda(cudaMemcpy(e->rope[l], cs.data(), cs.size() * sizeof(float2), cudaMemcpyHostToDevice), "rope table"));
+    }
+    TRY(alloc_workspace(e));
+    e->p_wqkv_d.resize(L); e->p_wo.resize(L); e->p_w1_d.resize(L); e->p_w2.resize(L);
+    for (int l = 0; l < L; ++l) {
+        TRY(make_tmap_2d(&e->p_wqkv_d[l], e->wqkv_d[l], 2, 3 * H, H, static_cast<uint64_t>(H) * 2, GEMM2_B_ROWS, 64));
+        TRY(make_tmap_2d(&e->p_wo[l], e->wo[l], 2, H, H, static_cast<uint64_t>(H) * 2, GEMM2_B_ROWS, 64));
+        TRY(make_tmap_2d(&e->p_w1_d[l], e->w1_d[l], 2, 2 * I, H, static_cast<uint64_t>(H) * 2, GEMM2_B_ROWS, 64));
+        TRY(make_tmap_2d(&e->p_w2[l], e->w2[l], 2, H, I, static_cast<uint64_t>(I) * 2, GEMM2_B_ROWS, 64));
+    }
+    TRY(check_cuda(cudaDeviceSynchronize(), "encoder_create_modernbert sync"));
 #undef TRY
     *out = e;
     return AC_OK;
@@ -1136,6 +1461,73 @@ using EpiGeluDefer16 = EpiLinear<1, true, false, true, 64>; // GELU(r (acc - mu 
 template <class Epi, int kEpiWarps = GEMM_EPI_WARPS>
 static int launch_linear(const CUtensorMap &ta, const CUtensorMap &tb, int M, int N, int K, const Epi &epi, cudaStream_t s) {
     return launch_gemm_tc2<Epi, false, GEMM_KIND_F16, kEpiWarps>(ta, tb, M, N, K, epi, s);
+}
+
+// ModernBERT forward (pre-LN): e->x holds the residual stream x (fp32); every LayerNorm is materialised as the fp16 A operand
+// of the projection that consumes it, so the projections run on plain fp16 weights with bias epilogues.  (The deferred form
+// of the post-LN path folds LN into the consumer as r (acc - mu c1) + c0; on a pre-LN stream, whose row mean grows with
+// depth, both that difference and the E[y^2] - mu^2 variance cancel, and the materialised LayerNorm costs one extra
+// read of x and fp16 write per half layer.)
+static int forward_modernbert(ac_encoder *e, const int32_t *ids, const int32_t *mask, int B, int S, float *out_unit_cls,
+                              cudaStream_t s) {
+    const ac_encoder_config &c = e->cfg;
+    const int H = c.hidden, I = c.intermediate, M = B * S;
+    const int S_pad = (S + 7) / 8 * 8;
+    const int wpb = 8;
+    const int row_blocks = (M + wpb - 1) / wpb;
+    int rc;
+    // layer 0's attn_norm is the identity: the normalised embeddings are both the stream and the first A operand
+    embed_norm_kernel<<<row_blocks, wpb * 32, 0, s>>>(ids, e->word, e->emb_ln_w, e->emb_ln_b, c.ln_eps, M, H, c.vocab, e->x, e->xh);
+    AC_LAUNCH_CHECK();
+    for (int l = 0; l < c.layers; ++l) {
+        if (l > 0) {
+            layernorm_kernel<<<row_blocks, wpb * 32, 0, s>>>(e->x, e->attn_nw[l], e->attn_nb[l], c.ln_eps, M, H, nullptr, e->xh);
+            AC_LAUNCH_CHECK();
+        }
+        EpiQKVRope eq{e->bqkv[l], e->qk, e->vT, e->rope[l], M, H, S, S_pad};
+        if ((rc = launch_linear(e->m_xh, e->p_wqkv_d[l], M, 3 * H, H, eq, s))) return rc;
+        if ((rc = launch_attention(e, mask, B, S, s, e->window[l]))) return rc;
+        if (l == c.layers - 1 && c.cls_only && static_cast<size_t>(B) <= e->Bc) {
+            // ---- CLS-only tail (classifier.py:1272 pools row 0): Wo + residual, mlp_norm, GeGLU, mlp.Wo + residual and
+            // final_norm on the B CLS rows
+            const int cb = (B + wpb - 1) / wpb;
+            gather_cls_kernel<<<cb, wpb * 32, 0, s>>>(e->ctx, e->x, B, S, H, e->ctx_cls, e->x_cls);
+            AC_LAUNCH_CHECK();
+            EpiResid eo{e->bo[l], e->x_cls, e->tmp_cls, B, H, H, 0, nullptr, 0, 0, 0, 0};
+            if ((rc = launch_linear(e->m_ctx_cls, e->p_wo[l], B, H, H, eo, s))) return rc;
+            layernorm_kernel<<<cb, wpb * 32, 0, s>>>(e->tmp_cls, e->mlp_nw[l], e->mlp_nb[l], c.ln_eps, B, H, nullptr, e->xh_cls);
+            AC_LAUNCH_CHECK();
+            EpiGeGLU eg{e->bi[l], e->ffn_cls, B, 2 * I, I};
+            if ((rc = launch_linear(e->m_xh_cls, e->p_w1_d[l], B, 2 * I, H, eg, s))) return rc;
+            EpiResid e2{e->b2[l], e->tmp_cls, e->x_cls, B, H, H, 0, nullptr, 0, 0, 0, 0};
+            if ((rc = launch_linear(e->m_ffn_cls, e->p_w2[l], B, H, I, e2, s))) return rc;
+            layernorm_kernel<<<cb, wpb * 32, 0, s>>>(e->x_cls, e->final_nw, e->final_nb, c.ln_eps, B, H, e->tmp_cls, nullptr);
+            AC_LAUNCH_CHECK();
+            if ((rc = launch_cls_normalize(e->tmp_cls, B, 1, H, out_unit_cls, s))) return rc;
+            e->last_B = B;
+            e->last_S = S;
+            e->last_cls_only = true;
+            return AC_OK;
+        }
+        // x' = x + Wo(ctx) into e->tmp, then x = x' + mlp.Wo(GeGLU(Wi(mlp_norm(x')))) back into e->x
+        EpiResid eo{e->bo[l], e->x, e->tmp, M, H, H, 0, nullptr, 0, 0, 0, 0};
+        if ((rc = launch_linear(e->m_ctx, e->p_wo[l], M, H, H, eo, s))) return rc;
+        layernorm_kernel<<<row_blocks, wpb * 32, 0, s>>>(e->tmp, e->mlp_nw[l], e->mlp_nb[l], c.ln_eps, M, H, nullptr, e->xh);
+        AC_LAUNCH_CHECK();
+        EpiGeGLU eg{e->bi[l], e->ffn, M, 2 * I, I};
+        if ((rc = launch_linear(e->m_xh, e->p_w1_d[l], M, 2 * I, H, eg, s))) return rc;
+        EpiResid e2{e->b2[l], e->tmp, e->x, M, H, H, 0, nullptr, 0, 0, 0, 0};
+        if ((rc = launch_linear(e->m_ffn, e->p_w2[l], M, H, I, e2, s))) return rc;
+    }
+    // full hidden state (cls_only = 0): final_norm on every row
+    layernorm_kernel<<<row_blocks, wpb * 32, 0, s>>>(e->x, e->final_nw, e->final_nb, c.ln_eps, M, H, e->tmp, nullptr);
+    AC_LAUNCH_CHECK();
+    if ((rc = launch_cls_normalize(e->tmp, B, S, H, out_unit_cls, s))) return rc;
+    e->last_B = B;
+    e->last_S = S;
+    e->last_cls_only = false;
+    e->last_hidden = e->tmp;
+    return AC_OK;
 }
 
 extern "C" int ac_encoder_forward_cls(ac_encoder *e, const int32_t *ids, const int32_t *mask, const int32_t *type_ids,
@@ -1162,6 +1554,7 @@ extern "C" int ac_encoder_forward_cls(ac_encoder *e, const int32_t *ids, const i
             return rc;
         e->vt_B = B; e->vt_S = S;
     }
+    if (c.arch == AC_ARCH_MODERNBERT) return forward_modernbert(e, ids, mask, B, S, out_unit_cls, s);
     const int wpb = 8;
     const int row_blocks = (M + wpb - 1) / wpb;
     const int nparts = H / 128;

@@ -1,6 +1,6 @@
 """Synthetic workloads of BASELINE.json / SURVEY.md section 8(d), shared by bench.py, __graft_entry__.smoke() and tests.
 
-No network, no datasets, no checkpoints: seeded random-init bert-base architecture, synthetic token ids,
+No network, no datasets, no checkpoints: seeded random-init bert-base (and ModernBERT-base) architecture, synthetic token ids,
 class-structured synthetic prototype rows (row j belongs to class j mod C)."""
 from __future__ import annotations
 
@@ -15,6 +15,26 @@ def bert_base_state_dict(seed: int = 1234, **cfg_over):
     m = BertModel(cfg, add_pooling_layer=False)
     m.eval()
     return m, cfg
+
+
+def modernbert_base_state_dict(seed: int = 1234, **cfg_over):
+    """HF ModernBertModel(ModernBertConfig()) == ModernBERT-base architecture (22 layers, H 768, I 1152, vocab 50368),
+    random init under torch.manual_seed(seed)."""
+    from transformers import ModernBertConfig, ModernBertModel
+    torch.manual_seed(seed)
+    cfg = ModernBertConfig(**cfg_over)
+    m = ModernBertModel(cfg)
+    m.eval()
+    return m, cfg
+
+
+def modernbert_synthetic_ids(B: int, S: int, vocab: int = 50368, seed: int = 7) -> torch.Tensor:
+    """uniform in [1000, vocab), CLS = 50281 first, SEP = 50282 last, no padding; int32 [B,S] on the host."""
+    g = torch.Generator().manual_seed(seed)
+    ids = torch.randint(min(1000, vocab - 1), vocab, (B, S), generator=g, dtype=torch.int64)
+    ids[:, 0] = min(50281, vocab - 1)
+    ids[:, -1] = min(50282, vocab - 1)
+    return ids.to(torch.int32)
 
 
 def synthetic_ids(B: int, S: int, vocab: int = 30522, seed: int = 7) -> torch.Tensor:

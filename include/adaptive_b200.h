@@ -195,7 +195,7 @@ int ac_ewc_penalty(const ac_head_params *p, const ac_head_params *fisher, const 
  * Stage E -- encoder.  Replaces `self.model(**inputs).last_hidden_state[:,0,:]` + F.normalize at
  *   src/adaptive_classifier/classifier.py:1271-1275 (HF BertModel / RobertaModel forward).
  * ------------------------------------------------------------------------------------------ */
-enum { AC_ARCH_BERT = 0, AC_ARCH_ROBERTA = 1 };
+enum { AC_ARCH_BERT = 0, AC_ARCH_ROBERTA = 1, AC_ARCH_MODERNBERT = 2 };
 enum {
     AC_PREC_TF32 = 0,   /* tcgen05 kind::tf32 on fp32 storage (kNN coarse pass, ac_linear_tc tests) */
     AC_PREC_F16 = 1     /* tcgen05 kind::f16 with fp16 operands (RNE from fp32; same 10-bit mantissa as tf32),
@@ -229,6 +229,39 @@ typedef struct ac_encoder ac_encoder;
 /* copies + repacks the weights (fused QKV, operand rounding) and allocates the activation workspace */
 int ac_encoder_create(const ac_encoder_config *cfg, const ac_encoder_weights *w, ac_encoder **out);
 int ac_encoder_destroy(ac_encoder *enc);
+
+/* ModernBERT (the reference's tests use answerdotai/ModernBERT-base: tests/test_order_independence.py:10,
+ * tests/test_confidence_consistency.py:14), HF transformers models/modernbert/modeling_modernbert.py:
+ *   embeddings LayerNorm(tok_embeddings[ids]) :52-71; pre-LN block x += Wo(attn(attn_norm(x))), x += mlp(mlp_norm(x))
+ *   :313-343 (attn_norm = identity in layer 0); fused Wqkv [3H, H] with RoPE (rotate_half, pairs d and d + 32 of each
+ *   64-wide head) :204-310; GeGLU mlp Wo(gelu_erf(input) * gate) with input, gate = Wi(x).chunk(2) :74-91; final_norm.
+ * Sliding layers see key k from query q iff |q - k| <= window (inclusive, masking_utils.py:121-131).  Creates the same
+ * ac_encoder handle as ac_encoder_create: forward_cls, last_hidden, destroy and the pipeline take it unchanged, and
+ * forward_cls ignores type_ids for it (ModernBERT has no token types).  S <= 512, head_dim 64. */
+typedef struct {
+    int layers, hidden, heads;
+    int intermediate;        /* I: Wi has 2I rows, mlp.Wo has I columns; multiple of 64 */
+    int vocab;
+    float norm_eps;
+    int precision;           /* AC_PREC_F16 */
+    int max_tokens;
+    int cls_only;            /* as in ac_encoder_config */
+    const int *window;       /* host array [layers]: key window of each layer (config.sliding_window), 0 = global */
+    const float *rope_theta; /* host array [layers]: rope_theta of each layer's type */
+} ac_modernbert_config;
+
+/* device pointers to the HF state_dict tensors (fp32, [out, in]); a NULL bias (or NULL bias array) means zero */
+typedef struct {
+    const float *tok_emb, *emb_norm_w, *emb_norm_b;
+    /* arrays of `layers` device pointers each (host arrays); attn_norm_w[0] / attn_norm_b[0] are ignored (NULL) */
+    const float *const *attn_norm_w, *const *attn_norm_b;
+    const float *const *Wqkv, *const *Wqkv_b, *const *Wo, *const *Wo_b;
+    const float *const *mlp_norm_w, *const *mlp_norm_b;
+    const float *const *Wi, *const *Wi_b, *const *mlp_Wo, *const *mlp_Wo_b;
+    const float *final_norm_w, *final_norm_b;
+} ac_modernbert_weights;
+
+int ac_encoder_create_modernbert(const ac_modernbert_config *cfg, const ac_modernbert_weights *w, ac_encoder **out);
 
 /* ids[B,S] int32 token ids, mask[B,S] int32 (1 keep / 0 pad; NULL = all ones), type_ids nullable.
  * out_unit_cls[B,H] = L2-normalised (eps 1e-12) CLS row of the last hidden state. */
