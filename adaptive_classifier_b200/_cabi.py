@@ -31,7 +31,7 @@ EXPORTS = [
     "ac_knn_workspace_bytes", "ac_knn_l2_topk", "ac_knn_make_shadow", "ac_row_sqnorm", "ac_topk_merge", "ac_proto_scores",
     "ac_segment_mean", "ac_memory_append_prune",
     "ac_head_forward", "ac_head_train_workspace_bytes", "ac_head_train_step", "ac_head_train_epoch", "ac_head_phase_timing", "ac_head_train_plan", "ac_head_grad", "ac_ewc_penalty",
-    "ac_encoder_create", "ac_encoder_create_modernbert", "ac_encoder_destroy", "ac_encoder_forward_cls", "ac_encoder_last_hidden", "ac_linear_tc",
+    "ac_encoder_create", "ac_encoder_create_modernbert", "ac_encoder_destroy", "ac_encoder_forward_cls", "ac_encoder_last_hidden", "ac_linear_tc", "ac_attention",
     "ac_proto_class_scores", "ac_proto_class_scores_n", "ac_blend_dense", "ac_topk_desc_workspace_bytes", "ac_topk_desc", "ac_blend_topk",
     "ac_pipeline_create", "ac_pipeline_destroy", "ac_pipeline_predict_device", "ac_pipeline_predict_host",
     "ac_pipeline_encode", "ac_pipeline_embeddings", "ac_pipeline_search_shard", "ac_pipeline_finish_sharded",
@@ -134,6 +134,7 @@ def load_library() -> ctypes.CDLL:
     L.ac_encoder_last_hidden.argtypes = [c_void_p, c_void_p, c_int64, c_void_p]
     L.ac_linear_tc.argtypes = [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int,
                                c_int, c_int, c_void_p]
+    L.ac_attention.argtypes = [c_void_p, c_int64, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p]
     L.ac_proto_class_scores.argtypes = [c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p, c_void_p]
     L.ac_proto_class_scores_n.argtypes = [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p]
     L.ac_blend_dense.argtypes = [c_void_p, c_void_p, c_int, c_void_p, c_int, c_int, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p]
@@ -445,6 +446,24 @@ def linear_tc(X, W, bias, residual=None, epi: int = 0, round_out: bool = False, 
     check(L.ac_linear_tc(X.data_ptr(), W.data_ptr(), ptr(bias), ptr(residual), Y.data_ptr(), M, N, K, epi,
                          1 if round_out else 0, prec, 1 if out_half else 0, stream_ptr()), "ac_linear_tc")
     return Y
+
+
+def attention(qk: torch.Tensor, vT: torch.Tensor, mask: Optional[torch.Tensor], B: int, S: int, heads: int,
+              window: int = 0) -> torch.Tensor:
+    """The encoder's attention on caller buffers (see ac_attention): qk fp16 [rows >= B*S, 2H], vT fp16 [B*H, roundup(S, 8)],
+    mask int32 [B, S] or None, window 0 = global -> ctx fp16 [B*S, H].  ctx starts as NaN, so a row the kernels never
+    write cannot pass for a result."""
+    L = load_library()
+    H = 64 * heads
+    assert qk.is_cuda and qk.dtype == torch.float16 and qk.is_contiguous() and qk.dim() == 2 and qk.shape[1] == 2 * H
+    assert vT.is_cuda and vT.dtype == torch.float16 and vT.is_contiguous() and tuple(vT.shape) == (B * H, (S + 7) // 8 * 8)
+    if mask is not None:
+        mask = mask.to(device=qk.device, dtype=torch.int32).contiguous()
+        assert tuple(mask.shape) == (B, S)
+    ctx = torch.full((B * S, H), float("nan"), dtype=torch.float16, device=qk.device)
+    check(L.ac_attention(qk.data_ptr(), qk.shape[0], vT.data_ptr(), ptr(mask), B, S, heads, window, ctx.data_ptr(),
+                         stream_ptr()), "ac_attention")
+    return ctx
 
 
 def distilbert_to_bert_state_dict(sd: dict, c):

@@ -1162,10 +1162,11 @@ static int launch_cls_normalize(const float *x, int B, int S, int H, float *out,
     return AC_OK;
 }
 
-// softmax(Q K^T / 8 + mask) V out of e->qk / e->vT into e->ctx
-static int launch_attention(ac_encoder *e, const int32_t *mask, int B, int S, cudaStream_t s, int window = 0) {
-    const ac_encoder_config &c = e->cfg;
-    const int H = c.hidden;
+// softmax(Q K^T / 8 + mask) V into ctx [B*S, H]: tqk is the 128-row-box map of qk [rows, 2H], tvt the 64 x 64-box map of
+// vT [(b, h, d), S_pad].  The one dispatch of the encoder and of ac_attention (S <= 128 / long kernel, window or global).
+static int launch_attention(const CUtensorMap &tqk, const CUtensorMap &tvt, const int32_t *mask, int B, int S, int heads,
+                            __half *ctx, cudaStream_t s, int window = 0) {
+    const int H = heads * 64;
     // per-device: the attribute is a property of the (function, device) pair
     static bool att_attr[64] = {};
     int dev = 0;
@@ -1180,19 +1181,16 @@ static int launch_attention(ac_encoder *e, const int32_t *mask, int B, int S, cu
     // algorithmic flops of softmax(QK^T)V at the true sequence length (the 128-wide tile does more)
     // a window that covers the whole sequence is global attention
     const bool win = window > 0 && window < S - 1;
-    const int slot = prof_begin(PROF_ATTENTION, 4.0 * B * c.heads * static_cast<double>(S) * S * 64, 0.0, s);
-    const dim3 grid_long(B * c.heads, (S + 127) / 128);
+    const int slot = prof_begin(PROF_ATTENTION, 4.0 * B * heads * static_cast<double>(S) * S * 64, 0.0, s);
+    const dim3 grid_long(B * heads, (S + 127) / 128);
     if (S <= 128 && win)
-        attention_kernel<true><<<B * c.heads, ATT_THREADS, ATT_SMEM, s>>>(e->m_qk_att, e->m_vt_att, mask, B, S, c.heads, H, e->ctx,
-                                                                          window);
+        attention_kernel<true><<<B * heads, ATT_THREADS, ATT_SMEM, s>>>(tqk, tvt, mask, B, S, heads, H, ctx, window);
     else if (S <= 128)
-        attention_kernel<false><<<B * c.heads, ATT_THREADS, ATT_SMEM, s>>>(e->m_qk_att, e->m_vt_att, mask, B, S, c.heads, H, e->ctx, 0);
+        attention_kernel<false><<<B * heads, ATT_THREADS, ATT_SMEM, s>>>(tqk, tvt, mask, B, S, heads, H, ctx, 0);
     else if (win)
-        attention_long_kernel<true><<<grid_long, ATT_THREADS, ATTL_SMEM, s>>>(e->m_qk_att, e->m_vt_att, mask, B, S, c.heads, H,
-                                                                               e->ctx, window);
+        attention_long_kernel<true><<<grid_long, ATT_THREADS, ATTL_SMEM, s>>>(tqk, tvt, mask, B, S, heads, H, ctx, window);
     else
-        attention_long_kernel<false><<<grid_long, ATT_THREADS, ATTL_SMEM, s>>>(e->m_qk_att, e->m_vt_att, mask, B, S, c.heads, H,
-                                                                                e->ctx, 0);
+        attention_long_kernel<false><<<grid_long, ATT_THREADS, ATTL_SMEM, s>>>(tqk, tvt, mask, B, S, heads, H, ctx, 0);
     prof_end(slot, s);
     AC_LAUNCH_CHECK();
     return AC_OK;
@@ -1245,7 +1243,10 @@ static int alloc_workspace(ac_encoder *e) {
     fill_value_kernel<<<(H + 255) / 256, 256>>>(e->ones, H, 1.f);
     fill_value_kernel<<<(H + 255) / 256, 256>>>(e->zeros, H, 0.f);
     WS(check_cuda(cudaGetLastError(), "deferred-LayerNorm constants"));
-    e->vt_elems = 2 * T * H;     // (b, h, d) rows x S_pad keys, S_pad = roundup(S, 8) <= 2*S for S >= 8
+    // V^T: (b, h, d) rows x S_pad keys, S_pad = roundup(S, 8) (TMA row pitch: 16 bytes).  Sized for every call forward_cls
+    // accepts (B*S <= max_tokens): B*S_pad <= floor(max_tokens / S) * roundup(S, 8), largest at S = 1 (8 * max_tokens); for
+    // S >= 8 it stays below 2 * max_tokens.
+    e->vt_elems = 8 * static_cast<size_t>(e->cfg.max_tokens) * H;
     WS(dev_alloc(e, &e->x, T * H));
     WS(dev_alloc(e, &e->tmp, T * H));
     WS(dev_alloc(e, &e->xh, T * H));
@@ -1486,7 +1487,7 @@ static int forward_modernbert(ac_encoder *e, const int32_t *ids, const int32_t *
         }
         EpiQKVRope eq{e->bqkv[l], e->qk, e->vT, e->rope[l], M, H, S, S_pad};
         if ((rc = launch_linear(e->m_xh, e->p_wqkv_d[l], M, 3 * H, H, eq, s))) return rc;
-        if ((rc = launch_attention(e, mask, B, S, s, e->window[l]))) return rc;
+        if ((rc = launch_attention(e->m_qk_att, e->m_vt_att, mask, B, S, c.heads, e->ctx, s, e->window[l]))) return rc;
         if (l == c.layers - 1 && c.cls_only && static_cast<size_t>(B) <= e->Bc) {
             // ---- CLS-only tail (classifier.py:1272 pools row 0): Wo + residual, mlp_norm, GeGLU, mlp.Wo + residual and
             // final_norm on the B CLS rows
@@ -1571,7 +1572,7 @@ extern "C" int ac_encoder_forward_cls(ac_encoder *e, const int32_t *ids, const i
     for (int l = 0; l < c.layers; ++l) {
         EpiQKVDefer eq{e->c0qkv[l], nullptr, e->qk, M, 3 * H, 2 * H, 0, e->vT, 2 * H, S, S_pad, H, e->c1qkv[l], st_in};
         if ((rc = launch_linear(e->m_xh, e->p_wqkv_d[l], M, 3 * H, H, eq, s))) return rc;
-        if ((rc = launch_attention(e, mask, B, S, s))) return rc;
+        if ((rc = launch_attention(e->m_qk_att, e->m_vt_att, mask, B, S, c.heads, e->ctx, s))) return rc;
         if (l == c.layers - 1 && c.cls_only && static_cast<size_t>(B) <= e->Bc) {
             // ---- CLS-only tail of the last layer (classifier.py:1272 pools row 0): M = B rows.  LN_pending is materialised on
             // the CLS rows and the tail runs on ordinary LayerNorm kernels and the plain (not gamma-scaled) FFN1 weight
@@ -1633,6 +1634,24 @@ extern "C" int ac_encoder_last_hidden(ac_encoder *e, float *out, int64_t n_float
     AC_CUDA(cudaMemcpyAsync(out, e->last_hidden ? e->last_hidden : e->x, n_floats * sizeof(float), cudaMemcpyDeviceToDevice,
                             static_cast<cudaStream_t>(stream)));
     return AC_OK;
+}
+
+// the encoder's attention exposed for parity tests: the tensor maps the encoder caches, built over caller buffers, and the
+// encoder's own dispatch
+extern "C" int ac_attention(const void *qk, int64_t qk_rows, const void *vT, const int32_t *mask, int B, int S, int heads,
+                            int window, void *ctx, ac_stream_t stream) {
+    AC_REQUIRE(qk && vT && ctx, "ac_attention: null argument");
+    AC_REQUIRE(B > 0 && S > 0 && S <= 512 && heads > 0 && window >= 0, "ac_attention: B=%d S=%d heads=%d window=%d", B, S, heads,
+               window);
+    AC_REQUIRE(qk_rows >= static_cast<int64_t>(B) * S, "ac_attention: qk has %lld rows, B*S = %lld", (long long)qk_rows,
+               static_cast<long long>(B) * S);
+    int rc = ac_device_check();
+    if (rc) return rc;
+    const int H = heads * 64, S_pad = (S + 7) / 8 * 8;
+    CUtensorMap tqk, tvt;
+    if ((rc = make_tmap_2d(&tqk, qk, 2, static_cast<uint64_t>(qk_rows), 2 * H, static_cast<uint64_t>(2 * H) * 2, 128, 64))) return rc;
+    if ((rc = make_tmap_2d(&tvt, vT, 2, static_cast<uint64_t>(B) * H, S_pad, static_cast<uint64_t>(S_pad) * 2, 64, 64))) return rc;
+    return launch_attention(tqk, tvt, mask, B, S, heads, static_cast<__half *>(ctx), static_cast<cudaStream_t>(stream), window);
 }
 
 // generic tensor-core linear exposed for parity tests / roofline measurement (the encoder's CTA-pair GEMM with a plain epilogue).

@@ -280,6 +280,17 @@ int ac_encoder_last_hidden(ac_encoder *enc, float *out, int64_t n_floats, ac_str
 int ac_linear_tc(const void *X, const void *W, const float *bias, const float *residual, void *Y,
                  int M, int N, int K, int epi, int round_out, int precision, int out_half, ac_stream_t stream);
 
+/* the encoder's attention, exposed for parity tests; it runs the same dispatch ac_encoder_forward_cls uses (S <= 128 kernel or
+ * the 128-query-block kernel, windowed when 0 < window < S - 1).  Per (sequence b, head h), H = 64 * heads:
+ *   ctx[b*S + q, 64h + :] = sum_k P[q,k] V[k] / sum_k P[q,k],  P[q,k] = exp((Q[q].K[k] - max) / 8) over the keys k < S with
+ *   mask[b,k] != 0 and, when windowed, |q - k| <= window; a query row with no such key gets zeros.
+ * qk  fp16 [qk_rows, 2H]: Q in columns [0, H), K in [H, 2H) (the encoder's layout); qk_rows >= B*S.  The kernels read whole
+ *     128-row tiles, so rows of neighbouring sequences and rows past B*S are loaded and must be ignored.
+ * vT  fp16 [(b, h, d), S_pad]: V transposed per (sequence, head), S_pad = roundup(S, 8); keys S .. S_pad-1 are ignored.
+ * mask int32 [B, S] nullable (1 keep / 0 pad), window 0 = global, ctx fp16 [B*S, H], S <= 512. */
+int ac_attention(const void *qk, int64_t qk_rows, const void *vT, const int32_t *mask, int B, int S, int heads, int window,
+                 void *ctx, ac_stream_t stream);
+
 /* ------------------------------------------------------------------------------------------
  * predict_batch() glue on the device (classifier.py:1329-1384) and the end-to-end pipeline.
  * ------------------------------------------------------------------------------------------ */

@@ -18,7 +18,7 @@ Pinned against HF ModernBertModel (eager and sdpa) by tests/test_modernbert_cpu.
 from __future__ import annotations
 
 import math
-from typing import Dict, List, Tuple
+from typing import Callable, Dict, List, Optional, Tuple
 
 import torch
 
@@ -33,8 +33,8 @@ def _ln(x: Tensor, sd: Dict[str, Tensor], name: str, eps: float) -> Tensor:
     return y + b if b is not None else y
 
 
-def _lin(x: Tensor, sd: Dict[str, Tensor], name: str) -> Tensor:
-    y = x @ sd[name + ".weight"].t()
+def _lin(x: Tensor, sd: Dict[str, Tensor], name: str, r: Callable[[Tensor], Tensor] = lambda t: t) -> Tensor:
+    y = r(x) @ r(sd[name + ".weight"]).t()
     b = sd.get(name + ".bias")
     return y + b if b is not None else y
 
@@ -66,9 +66,12 @@ def _rotate_half(x: Tensor) -> Tensor:
 
 
 def modernbert_forward_cls(sd: Dict[str, Tensor], ids: Tensor, mask, cfg, return_hidden: bool = False,
-                           inclusive_window: bool = True):
+                           inclusive_window: bool = True, round_fn: Optional[Callable[[Tensor], Tensor]] = None):
     """unit-norm CLS rows fp32 [B, H] (and the final-normed hidden state [B, S, H] with return_hidden).
-    inclusive_window=False restates the off-by-one variant |q - k| < window (only to show that tests can see it)."""
+    inclusive_window=False restates the off-by-one variant |q - k| < window (only to show that tests can see it).
+    round_fn (as in oracle/encoder_oracle.py) is applied to both operands of every matrix product -- the linears, q k^T after
+    RoPE and P V with the normalised P -- to restate the B200 path's fp16 operand rounding."""
+    r = round_fn if round_fn is not None else (lambda t: t)
     B, S = ids.shape
     if mask is None:
         mask = torch.ones_like(ids)
@@ -84,7 +87,7 @@ def modernbert_forward_cls(sd: Dict[str, Tensor], ids: Tensor, mask, cfg, return
     for l in range(cfg.num_hidden_layers):
         p = f"layers.{l}."
         h = x if l == 0 else _ln(x, sd, p + "attn_norm", eps)
-        qkv = _lin(h, sd, p + "attn.Wqkv").view(B, S, 3, nh, dh)
+        qkv = _lin(h, sd, p + "attn.Wqkv", r).view(B, S, 3, nh, dh)
         q, k, v = (qkv[:, :, j].transpose(1, 2) for j in range(3))  # [B, nh, S, dh]
         cos, sin = rope_cos_sin(thetas[l], S, dh)
         q = q * cos + _rotate_half(q) * sin
@@ -93,14 +96,14 @@ def modernbert_forward_cls(sd: Dict[str, Tensor], ids: Tensor, mask, cfg, return
         if wins[l]:
             near = (dist <= wins[l]) if inclusive_window else (dist < wins[l])
             vis = vis & near[None, None]
-        scores = (q @ k.transpose(-1, -2)) * dh ** -0.5
+        scores = (r(q) @ r(k).transpose(-1, -2)) * dh ** -0.5
         scores = scores.masked_fill(~vis, neg)
-        ctx = torch.softmax(scores, dim=-1) @ v
+        ctx = r(torch.softmax(scores, dim=-1)) @ r(v)
         ctx = ctx.transpose(1, 2).reshape(B, S, H)
-        x = x + _lin(ctx, sd, p + "attn.Wo")
+        x = x + _lin(ctx, sd, p + "attn.Wo", r)
         h = _ln(x, sd, p + "mlp_norm", eps)
-        a, g = _lin(h, sd, p + "mlp.Wi").chunk(2, dim=-1)
-        x = x + _lin(_gelu_erf(a) * g, sd, p + "mlp.Wo")
+        a, g = _lin(h, sd, p + "mlp.Wi", r).chunk(2, dim=-1)
+        x = x + _lin(_gelu_erf(a) * g, sd, p + "mlp.Wo", r)
     x = _ln(x, sd, "final_norm", eps)
     cls = x[:, 0, :]
     unit = cls / cls.norm(dim=1, keepdim=True).clamp_min(1e-12)

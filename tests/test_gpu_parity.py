@@ -455,7 +455,11 @@ def test_encoder_full_last_layer_and_hidden_state(cabi):
     b = enc_cls.forward_cls(ids.to(torch.int32).cuda()).cpu()
     assert (a - ref_cls).norm(dim=1).max() < 1e-3 and (b - ref_cls).norm(dim=1).max() < 1e-3
     assert (a - b).abs().max() < 1e-4            # CLS-only tail: LayerNorm materialised on B rows; full flow: deferred into the epilogues
-    assert (hid - ref_hidden).abs().max() < 2e-2 * ref_hidden.abs().max()
+    # per row: the CLS rows above carry the same fp16 operand rounding (||dq|| <= 2.5e-4 at 2 layers, precision study), and
+    # every other row goes through the same GEMMs and attention
+    rel = ((hid - ref_hidden).norm(dim=-1) / ref_hidden.norm(dim=-1)).max().item()
+    print(f"full hidden state: max row rel err {rel:.3e}")
+    assert rel < 1e-3, rel
     with pytest.raises(cabi.AdaptiveB200Error):
         enc_cls.last_hidden(B, S)
     enc_full.close(); enc_cls.close()
@@ -560,7 +564,10 @@ def test_encoder_with_nontrivial_layernorms_matches_oracle(cabi, layers, B, S, c
     if not cls_only:
         hidden = enc.last_hidden(B, S).cpu()
         keep = mask.bool()
-        assert (hidden.view(B, S, -1)[keep] - ref_hidden[keep]).abs().max() < 5e-3
+        d = hidden.view(B, S, -1)[keep] - ref_hidden[keep]
+        rel = (d.norm(dim=-1) / ref_hidden[keep].norm(dim=-1)).max().item()
+        print(f"nontrivial LayerNorms, full hidden state: max row rel err {rel:.3e}")
+        assert rel < 1e-3, rel                   # per valid row, as the CLS rows above (||dq|| < 1e-3)
     enc.close()
 
 
